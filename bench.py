@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — train-step images/sec of the GAN / VAE hot path on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ns|wgp|vae]   # this repo's CUDA path
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ns|wgp|vae|dcgan] [--dump-outputs DIR]   # this repo's CUDA path
   python bench.py --impl reference [--gpus N] ...                                # the reference's own CPU path
   torchrun --nproc-per-node N bench.py --gpus N ...                              # N > 1 (driver does this)
 
@@ -256,6 +256,29 @@ class Workload:
     def losses(self):
         return [float(v) for v in self.loss_buf.tolist()]
 
+    def outputs(self):
+        """What a caller of step() gets from it: the step's losses and the updated fp32 parameters, by name."""
+        eng = self.eng
+        out = {"losses": self.loss_buf}
+        if self.name == "dcgan":
+            for tag, net in (("G", eng.G), ("D", eng.D)):
+                out.update(("%s.%s" % (tag, n), net.view(n)) for n in net.names)
+        elif self.name == "vae":
+            out.update(eng.views())
+        else:
+            names = [m + s for m in ("G.linear", "G.generate", "D.linear", "D.discriminate") for s in (".weight", ".bias")]
+            out.update(zip(names, eng.views(0) + eng.views(1)))
+        return out
+
+
+def dump_outputs(wl, out_dir):
+    """wl.outputs() as out_dir/<name>.npy in float32 (at most 26 MB: the DCGAN's parameters), so that two builds can be
+    compared output for output on the same seeded inputs."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in wl.outputs().items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
 
 def make_pool(N, dev, rank):
     """device-resident synthetic dataset, 1 bit per pixel (binarised MNIST carries exactly that:
@@ -346,6 +369,8 @@ def run_ours(args):
     launches = gm_b200.launch_count(reset=True)
     value = B * world * args.steps / (ms * 1e-3)
     losses = wl.losses()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
 
     # ---- e2e: same step through the host-facing call, HOST (pinned) batches; the H2D
     # copy of each step's batch and the D2H read of its losses are inside the timed region
@@ -659,7 +684,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--headline-only", action="store_true", help="skip the other workloads / trainer / small-batch legs")
     ap.add_argument("--no-parity-mode", action="store_true", help="skip the split-precision leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's losses and updated "
+                                                         "parameters as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -260,3 +260,27 @@ def test_graph_replay_matches_host_driven_steps():
         assert torch.equal(eng.params[net], ref.params[net]), net
         assert torch.equal(eng.exp_avg_sq[net], ref.exp_avg_sq[net])
     assert torch.equal(eng.loss_buf, ref.loss_buf)
+
+
+def test_bench_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: the losses the JSON line reports for the last timed step and the updated parameters,
+    float32 .npy files; a second run with the same arguments reproduces them bit for bit."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    runs = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--headline-only",
+                              "--no-cpu", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-3000:]
+        line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+        runs.append((line, {f[:-len(".npy")]: np.load(d / f) for f in os.listdir(d)}))
+    line, arrs = runs[0]
+    names = [m + s for m in ("G.linear", "G.generate", "D.linear", "D.discriminate") for s in (".weight", ".bias")]
+    assert line["steps"] == 2 and sorted(arrs) == sorted(["losses"] + names)
+    assert all(a.dtype == np.float32 for a in arrs.values()) and sum(a.nbytes for a in arrs.values()) <= 64 << 20
+    assert arrs["G.generate.weight"].shape == (X, H) and arrs["D.discriminate.weight"].shape == (1, H)
+    np.testing.assert_array_equal(arrs["losses"], np.float32(line["losses_last_step"]))
+    for name, a in runs[1][1].items():
+        np.testing.assert_array_equal(a, arrs[name], err_msg=name)

@@ -89,11 +89,12 @@ def test_reference_made_checkpoints_load_into_the_dropin_modules():
         assert torch.equal(v, vsd[k]), k
 
 
-def test_dcgan_dropin_surface_without_a_gpu():
+def test_dcgan_dropin_surface_without_a_gpu(monkeypatch):
     """dc_gan.py mirrors the NSGAN class surface for the conv model the README recommends (README.md:68,96): usual DCGAN
     state_dict keys / shapes, the reference's attributes, and a loud failure instead of a CPU fallback."""
     import dc_gan
     from gm_b200 import GmError
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)     # the same refusal on a machine that has a GPU
     model = dc_gan.DCGAN(image_size=64 * 64 * 3, hidden_dim=16, z_dim=100)
     sd = model.state_dict()
     assert sd["G.l1.weight"].shape == (100, 128, 4, 4) and sd["G.l5.weight"].shape == (16, 3, 4, 4)
